@@ -347,6 +347,24 @@ def decode_bench(wl, gen=64):
     return res
 
 
+DUMP_ROWS = 1 << 15     # --dump-outputs: K and V rows of D=128 float32 -> 2 x 16 MiB
+
+
+def dump_outputs(wl, out_dir):
+    """Writes what the last timed step returned: every layer's compacted K and V cache ([Hq, k_l + W, D] bf16), their rows
+    concatenated over layers and heads ([sum_l Hq * (k_l + W), D]), as float32 (exact for bf16). Larger outputs are cut to
+    DUMP_ROWS rows at the same seeded positions for K and V, so two builds can be compared row for row."""
+    k = torch.cat([c.reshape(-1, wl.D) for c in wl.kc])
+    v = torch.cat([c.reshape(-1, wl.D) for c in wl.vc])
+    if k.shape[0] > DUMP_ROWS:
+        rows = torch.randperm(k.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values.to(k.device)
+        k, v = k[rows], v[rows]
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "k_cache.npy"), k.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "v_cache.npy"), v.float().cpu().numpy())
+
+
 def timed(fn, steps, barrier):
     barrier()
     torch.cuda.synchronize()
@@ -529,9 +547,9 @@ def whole_model_numbers(device, ctx=32768, budget=128, new_tokens=128, fused_rop
 
 
 def gpu_arm(args, rank, world, local):
-    from pyramidkv_b200 import _lib, build, ops
+    from pyramidkv_b200 import _lib, ops
     from pyramidkv_b200.kv_cluster import PyramidKVCluster
-    build.build()
+    _lib.lib()      # built by `python -m pyramidkv_b200.build`; the benchmark compiles nothing and writes nothing into the tree
     device = torch.device("cuda", local)
     torch.cuda.set_device(device)
     use_dist = world > 1
@@ -546,6 +564,8 @@ def gpu_arm(args, rank, world, local):
 
     sharded = world > 1 and args.workload.startswith("llama3-70b")
     if sharded:
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs is not available for the layer-sharded 70B run")
         return sharded_70b_arm(args, rank, world, device, barrier)
     wl = Workload(args.workload, device, args.score_kernel, args.kv_layout, args.method, args.layers)
     if args.profile_only:
@@ -567,6 +587,8 @@ def gpu_arm(args, rank, world, local):
     n0 = _lib.launch_count()
     ms_step = timed(wl.step, args.steps, barrier)
     launches = (_lib.launch_count() - n0) // args.steps
+    if args.dump_outputs and rank == 0 and wl.batch is None:
+        dump_outputs(wl, args.dump_outputs)
 
     # ---- the layer batch: all layers in one pass (what the patched forward runs with pkv_defer_eviction) ----
     ms_batch, batch_ms, launches_batch = None, {}, 0
@@ -576,6 +598,8 @@ def gpu_arm(args, rank, world, local):
         n0 = _lib.launch_count()
         ms_batch = timed(wl.batch.run, args.steps, barrier)
         launches_batch = (_lib.launch_count() - n0) // args.steps
+        if args.dump_outputs and rank == 0:        # before the stage timings below overwrite the caches
+            dump_outputs(wl, args.dump_outputs)
         for st in ("scores", "pool", "select"):
             wl.batch.run(st)
             batch_ms[st] = timed(lambda s=st: wl.batch.run(s), max(3, args.steps // 2), barrier)
@@ -770,7 +794,14 @@ def main():
     ap.add_argument("--sharded-70b", type=int, default=1, help="N>1: after the weak-scaling numbers also run the layer-sharded Llama-3-70B arm (configs[4]) and report it under sharded_70b")
     ap.add_argument("--quick", type=int, default=0, help="1: only the resident-HBM eviction numbers (A/B runs; skips e2e, decode and the baselines - not a bench line)")
     ap.add_argument("--profile-only", action="store_true", help="run warmup+steps of the resident-HBM loop and exit (for ncu; prints no bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the compacted K/V caches of the last timed step to DIR/k_cache.npy and DIR/v_cache.npy (float32; "
+                         "a fixed seeded sample of rows when larger; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile_only):
+        ap.error("--dump-outputs writes the outputs of the timed GPU path: not with --impl reference or --profile-only")
     if args.budget or args.seq_len or args.layers or args.method != "pyramidkv":
         L, Hq, Hkv, D, S, B, W, ks, pool = WORKLOADS[args.workload]
         B = args.budget or B

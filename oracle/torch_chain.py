@@ -1,9 +1,9 @@
 """The reference's eviction op chain restated with stock PyTorch ops (runs on CPU or GPU).
 
 *** TEST / BASELINE INFRASTRUCTURE, NOT PRODUCT CODE. *** Used by tests (-m gpu: same-device comparison against
-the CUDA kernels) and by bench.py as the "reference op chain on this GPU" baseline. `/root/reference` does not
-exist on the GPU box, so the chain is restated here op for op; in the build container
-tests/test_torch_chain_vs_reference.py checks it bit-for-bit against the imported reference classes.
+the CUDA kernels) and by bench.py as the "reference op chain on this GPU" baseline. The reference is not a dependency
+of this repository, so the chain is restated here op for op; tests/test_torch_chain_vs_reference.py (and the
+`*_bit_identical_to_reference` tests) check it bit-for-bit against the outputs the reference classes recorded in tests/golden.
 
 Follows pyramidkv/pyramidkv_utils.py: budget :205-220; scoring :253-263 (== :317-327); pooling :264-269;
 top-k :270; gather + concat :271-282; H2O :544-575; StreamingLLM :607-619; repeat_kv :108-117; L2Norm :406-431.

@@ -108,29 +108,21 @@ def test_torch_chain_stable_rule_equals_oracle(oracle):
         assert torch.equal(kf, torch.cat(ks)) and torch.equal(vf, torch.cat(vs)) and lens == [int(c) + W for c in cap]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="build container only: needs the reference sources")
 def test_torch_chain_bit_identical_to_reference():
-    import contextlib, io, sys
-    sys.path.insert(0, GOLDEN_DIR)
-    from make_golden import load_reference
+    """The torch restatement reproduces what the reference's AdaKVCluster / HeadKVCluster returned on every golden case
+    (recorded by tests/golden/make_golden_adakv.py): scores, flat K/V (sha256) and head lengths."""
     from oracle import torch_chain as tc
-    ref = load_reference()
-    for seed, dt, scale in ((1, torch.bfloat16, 1.0), (2, torch.float16, 0.05)):
-        for (Hq, S, D, W, B, ks, pool, norm) in [(8, 700, 128, 32, 128, 7, "maxpool", True), (4, 400, 64, 8, 64, 5, "avgpool", False),
-                                                  (8, 100, 128, 32, 256, 7, "maxpool", True)]:
-            q, k, v = make_inputs(seed, Hq, Hq, S, D, dt, scale)
-            K, V, Q = k[None], v[None], q[None]
-            with contextlib.redirect_stdout(io.StringIO()):
-                c = ref.AdaKVCluster(window_size=W, kernel_size=ks, pooling=pool, max_capacity_prompt=B, floor=0.2, normalize=norm, layer_idx=0, num_hidden_layers=4)
-                ko, vo = c.update_kv(K, Q, V)
-            mk, mv, lens = tc.adakv_update_kv(K, Q, V, W, B, ks, pool, 0.2, norm)
-            assert torch.equal(ko, mk) and torch.equal(vo, mv) and lens == c.head_lens.tolist()
-            if B - W <= S - W:
-                hc = torch.tensor([[10, 3, 50, 7, 20, 1, 0, S + 40][:Hq]])     # the last budget exceeds the candidates: kept whole
-                c2 = ref.HeadKVCluster(window_size=W, kernel_size=ks, pooling=pool, max_capacity_prompt=B, layer_idx=0, num_hidden_layers=4, head_capacity=hc)
-                ko, vo = c2.update_kv(K, Q, V)
-                mk, mv, lens = tc.headkv_update_kv(K, Q, V, W, B, hc[0], ks, pool)
-                assert torch.equal(ko, mk) and torch.equal(vo, mv) and lens == c2.head_lens.tolist()
+    for name in ADAKV + ["adakv_pass_s100_b256_w32_bf16", "headkv_s1024_b128_w32_bf16"]:
+        z, m, dt, q, k, v = _load(name)
+        G = m["Hq"] // m["Hkv"]
+        K, V, Q = tc.repeat_kv(k[None], G), tc.repeat_kv(v[None], G), q[None]
+        assert torch.equal(tc.adakv_scores(K, Q, m["W"], m["kernel"], m["pooling"])[0].view(torch.int16), from_u16(z["score"], dt).view(torch.int16)), name
+        if m["kind"] == "adakv":
+            mk, mv, lens = tc.adakv_update_kv(K, Q, V, m["W"], m["B"], m["kernel"], m["pooling"], m["floor"], m["normalize"])
+        else:
+            mk, mv, lens = tc.headkv_update_kv(K, Q, V, m["W"], m["B"], torch.tensor(m["head_capacity"]), m["kernel"], m["pooling"])
+        assert sha256_of(mk) == m["sha_k_out"] and sha256_of(mv) == m["sha_v_out"], name
+        assert lens == z["head_lens"].tolist() and mk.shape[0] == m["rows"], name
 
 
 # ---------------- host mirror + plugin flow (test backend) ----------------
